@@ -9,8 +9,11 @@ BASELINE.json configs[1] shape (D_W_15K_V1, batch 5000) is measured in the same 
 `bootea_15k` block of the same JSON line (N = 1 only).
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--workload bootea_100k|bootea_15k]
+                    [--dump-outputs DIR]
 
-Prints ONE JSON line on rank 0.
+Prints ONE JSON line on rank 0.  With --dump-outputs, rank 0 also writes what the last timed step left for its caller
+(see dump_outputs) as DIR/<name>.npy; the inputs are seeded, so two builds run with the same arguments can be compared
+array for array.
 """
 import argparse
 import json
@@ -35,6 +38,9 @@ WORKLOADS = {
 }
 L2_FLUSH_BYTES = 512 << 20
 SHAPE_ENTITIES = {"15K": 15000, "100K": 100000}      # entities per KG (openea_b200/synth.py SHAPES)
+# --dump-outputs keeps under 64 MB: at dim 100 this many entity rows of weights + Adagrad slots are 52 MB
+DUMP_ENTITY_ROWS = 65536
+DUMP_ROW_SEED = 7
 
 
 def peaks():
@@ -134,6 +140,25 @@ def build_workload(wl, rank, device, world=1):
     steps_per_epoch = int(np.ceil(T / cfg["batch"]))
     return dict(cfg=cfg, arr=arr, ent=ent, rel=rel, kg1=kg1, kg2=kg2, tset=tset, trainer=trainer,
                 steps_per_epoch=steps_per_epoch, n_triples=T, n_triples_global=n_triples_global)
+
+
+def dump_outputs(out_dir, tr, last_step_loss):
+    """Writes what a caller of the timed path holds after its last step: that step's loss and the trained variables with
+    their Adagrad accumulators (raw, unnormalised rows).  Entity tables larger than DUMP_ENTITY_ROWS rows are sampled:
+    the same seeded, sorted row set on every run."""
+    import torch
+    os.makedirs(out_dir, exist_ok=True)
+    ent, rel = tr.ent, tr.rel
+    n = min(DUMP_ENTITY_ROWS, ent.rows)
+    rows = np.sort(np.random.default_rng(DUMP_ROW_SEED).choice(ent.rows, n, replace=False))
+    idx = torch.from_numpy(rows).to(ent.weight.device)
+    arrays = {"last_step_loss": np.array([last_step_loss], dtype=np.float64),
+              "entity_embeddings_sampled": ent.weight[idx, :ent.dim].cpu().numpy(),
+              "entity_adagrad_sampled": ent.state1[idx, :ent.dim].cpu().numpy(),
+              "relation_embeddings": rel.weight[:, :rel.dim].cpu().numpy(),
+              "relation_adagrad": rel.state1[:, :rel.dim].cpu().numpy()}
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a)
 
 
 def decode_dbg(dbg, n, t1, t2, k):
@@ -359,7 +384,7 @@ def probe_pipelined_e2e(args):
             got.append(pipe.collect((i - 1) % 2))
     got.append(pipe.collect(5 % 2))
     rel = max(abs(a - b) / max(1e-12, abs(b)) for a, b in zip(got, want))
-    K = max(8, args.steps)
+    K = args.steps
     torch.cuda.synchronize()
     t0 = time.perf_counter()
     for i in range(K):
@@ -501,11 +526,14 @@ def bench_triples(args, wl, rank, local_rank, world, device, full):
         dist.barrier()
     torch.cuda.synchronize()
     n_push0 = 0 if xchg is None else xchg.epoch
+    dump = full and rank == 0 and args.dump_outputs
     with ClockSampler(local_rank) as clocks:
         t_wall0 = time.perf_counter()
         for i in range(K):
             if not args.no_flush:
                 flush.fill_(float(i))   # L2 flush (not timed: outside the event pairs)
+            if dump and i == K - 1:
+                loss_before_last = tr.loss_dev.clone()      # outside the event pair, like the flush
             one_step(n_warm + i, evs[i])
         torch.cuda.synchronize()
         t_wall = time.perf_counter() - t_wall0
@@ -519,6 +547,8 @@ def bench_triples(args, wl, rank, local_rank, world, device, full):
         t = torch.tensor([total_ms], dtype=torch.float64, device=device)
         dist.all_reduce(t, op=dist.ReduceOp.MAX)
         total_ms = float(t.item())
+    if dump:          # before anything below steps the tables again
+        dump_outputs(args.dump_outputs, tr, float((tr.loss_dev - loss_before_last).item()))
     loss_val = tr.read_loss()
     value = world * n_pos_step * K / (total_ms * 1e-3)
 
@@ -624,25 +654,24 @@ def bench_triples(args, wl, rank, local_rank, world, device, full):
     from openea_b200 import engine as eng
     os.environ["OEA_FED_FUSED"] = "1"       # grouped scorer + row optimiser as one cooperative launch per step
     pipe = eng.FedHostPipeline(tr, 3 * (n_pos_h + n_neg_h) + 64)
-    Kp = max(K, 40)
     for rep in range(2):                    # rep 0 = warm-up
         if world > 1:
             dist.barrier()
         torch.cuda.synchronize()
         t0 = time.perf_counter()
-        for i in range(Kp):
+        for i in range(K):
             pipe.submit(i % 2, *host_batches[i % n_b])
             if i >= 1:
                 pipe.collect((i - 1) % 2)
-        pipe.collect((Kp - 1) % 2)
+        pipe.collect((K - 1) % 2)
         pipe_s = time.perf_counter() - t0
     os.environ.pop("OEA_FED_FUSED", None)
     if world > 1:
         t = torch.tensor([pipe_s], dtype=torch.float64, device=device)
         dist.all_reduce(t, op=dist.ReduceOp.MAX)
         pipe_s = float(t.item())
-    e2e = {"value": world * n_pos_h * Kp / pipe_s, "unit": unit, "h2d_bytes_per_step": 12 * (n_pos_h + n_neg_h),
-           "d2h_bytes_per_step": 8, "ms_per_step": 1e3 * pipe_s / Kp, "steps": Kp,
+    e2e = {"value": world * n_pos_h * K / pipe_s, "unit": unit, "h2d_bytes_per_step": 12 * (n_pos_h + n_neg_h),
+           "d2h_bytes_per_step": 8, "ms_per_step": 1e3 * pipe_s / K, "steps": K,
            "api": "oea_triple_step_fed_host_submit / _collect (pinned host index buffers, depth-2 pipeline, one cooperative launch per step)",
            "synchronous": sync_e2e}
     _phase("%s: e2e done" % wl)
@@ -700,7 +729,12 @@ def main():
     ap.add_argument("--no-flush", action="store_true", help="diagnostic only: keep L2 warm between timed steps (the number is NOT a valid bench value)")
     ap.add_argument("--probe-pipelined-e2e", action="store_true",
                     help="internal: measure the depth-2 pipelined host-index step in this process and print its JSON")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write the last step's loss and the trained tables (entity rows: a fixed "
+                         "seeded sample) as DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     if args.probe_pipelined_e2e:
         return probe_pipelined_e2e(args)
     rank = int(os.environ.get("RANK", "0"))

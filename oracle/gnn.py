@@ -18,12 +18,13 @@ import numpy as np
 import scipy.sparse as sp
 import torch
 
-REF_FILE = "/root/reference/src/openea/approaches/gcn_align.py"
+REF_DIR = os.path.join(os.environ.get("OPENEA_REFERENCE", ""), "src", "openea", "approaches")
+REF_FILE = os.path.join(REF_DIR, "gcn_align.py")
 
 
 def reference_gcn_utils():
     """(GCN_Utils class, load_attr function) compiled from the reference source; None if it is not present."""
-    if not os.path.exists(REF_FILE):
+    if not os.environ.get("OPENEA_REFERENCE") or not os.path.exists(REF_FILE):
         return None
     with open(REF_FILE) as f:
         tree = ast.parse(f.read())
@@ -77,13 +78,13 @@ def unit_train_step(support, W0, features, ill, gamma, k, negs, lr, dtype=torch.
 
 
 # ---- AliNet (approaches/alinet.py) — torch-CPU restatement with dense-free sparse ops (TF semantics unpinned) ----
-ALINET_REF_FILE = "/root/reference/src/openea/approaches/alinet.py"
+ALINET_REF_FILE = os.path.join(REF_DIR, "alinet.py")
 
 
 def reference_alinet_builders():
     """Namespace with the reference's own pure-Python/NumPy/pandas builders (AKG, enhance_triples, no_weighted_adj,
     generate_2hop_triples, remove_unlinked_triples, generate_rel_ht, …) compiled from its source; None if absent."""
-    if not os.path.exists(ALINET_REF_FILE):
+    if not os.environ.get("OPENEA_REFERENCE") or not os.path.exists(ALINET_REF_FILE):
         return None
     import math
     import time
@@ -152,12 +153,12 @@ def alinet_loss(params, outs, pos, neg, neg_margin, balance, hs, ts, rel_win, re
 
 
 # ---- RDGCN (approaches/rdgcn.py) — torch-CPU restatement (TF semantics unpinned) -------------------------------
-RDGCN_REF_FILE = "/root/reference/src/openea/approaches/rdgcn.py"
+RDGCN_REF_FILE = os.path.join(REF_DIR, "rdgcn.py")
 
 
 def reference_rdgcn_builders():
     """get_mat / rfunc of the reference compiled from its source (tf.SparseTensor stubbed to a tuple)."""
-    if not os.path.exists(RDGCN_REF_FILE):
+    if not os.environ.get("OPENEA_REFERENCE") or not os.path.exists(RDGCN_REF_FILE):
         return None
     import math
     import types

@@ -1,25 +1,25 @@
 """Import the REAL reference's NumPy modules (path (iii) + the sampler) with tensorflow / igraph stubbed.
 
-Only usable where /root/reference exists (the authoring container).  Used by tests/golden/make_golden.py to
-generate golden vectors and by CPU tests (skipped when the reference is absent) to pin oracle.finding.
-Nothing on the GPU box may import this at run time.  TEST INFRASTRUCTURE ONLY.
+Only usable where OPENEA_REFERENCE names a checkout of the original project.  Used by tests/golden/make_golden.py
+and by CPU tests run with OPENEA_REFERENCE set to record the golden results the tests compare with
+(tests/helpers.ReferenceRecord).  TEST INFRASTRUCTURE ONLY.
 """
 import importlib
 import os
 import sys
 import types
 
-REF_SRC = "/root/reference/src"
+REF_SRC = os.path.join(os.environ.get("OPENEA_REFERENCE", ""), "src")
 
 
 def available():
-    return os.path.isdir(os.path.join(REF_SRC, "openea"))
+    return bool(os.environ.get("OPENEA_REFERENCE")) and os.path.isdir(os.path.join(REF_SRC, "openea"))
 
 
 def load():
     """Returns a namespace with the reference modules: similarity, alignment, evaluation, batch, finder, read, util."""
     if not available():
-        raise RuntimeError("/root/reference is not present")
+        raise RuntimeError("set OPENEA_REFERENCE to a checkout of the original OpenEA")
     saved = {k: sys.modules.get(k) for k in ("tensorflow", "igraph", "openea")}
     saved_sub = {k: v for k, v in sys.modules.items() if k.startswith("openea.")}
     for k in saved_sub:

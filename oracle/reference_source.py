@@ -1,16 +1,16 @@
 """TEST INFRASTRUCTURE: pure-Python / NumPy / pandas helper functions of the reference compiled from its own source
-(selected top-level definitions only, so TensorFlow is never imported).  Available only where /root/reference exists
-(this container); tests that use it are skipped on the GPU box.  Nothing under openea_b200/ imports this."""
+(selected top-level definitions only, so TensorFlow is never imported).  Available only where OPENEA_REFERENCE names a
+checkout of the original project: tests call it to record their golden results.  Nothing under openea_b200/ imports this."""
 import ast
 import os
 
-REF_ROOT = "/root/reference/src/openea"
+REF_ROOT = os.path.join(os.environ.get("OPENEA_REFERENCE", ""), "src", "openea")
 
 
 def extract(rel_path, names, namespace):
     """Compile the top-level functions / classes `names` of REF_ROOT/rel_path into `namespace`; None if absent."""
     path = os.path.join(REF_ROOT, rel_path)
-    if not os.path.exists(path):
+    if not os.environ.get("OPENEA_REFERENCE") or not os.path.exists(path):
         return None
     with open(path) as f:
         tree = ast.parse(f.read())

@@ -1,8 +1,8 @@
 """CPU ORACLE end-to-end training loop for path (i) — TEST INFRASTRUCTURE ONLY.
 
 Restates BasicModel.run / launch_triple_training_1epo (models/basic_model.py:211-290) and the AlignE / BootEA
-configuration on the CPU: the reference's own Python sampler (modules/train/batch.py, imported from
-/root/reference when present, otherwise the behavioural port in openea_b200.modules.train.batch), the C oracle
+configuration on the CPU: the reference's own Python sampler (modules/train/batch.py, imported from the checkout
+OPENEA_REFERENCE names, otherwise the behavioural port in openea_b200.modules.train.batch), the C oracle
 step (dense TF semantics) and the NumPy evaluation.  Used to calibrate end-to-end accuracy (Hits@1) of the
 engine on the same synthetic KG: parity here is statistical (different RNG streams), not bit-wise.
 """

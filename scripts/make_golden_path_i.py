@@ -1,11 +1,11 @@
 """Generates tests/golden/path_i_reference_graphs.npz by EXECUTING the reference's own graph-definition code for path
 (i) — `_define_variables`, `_define_embed_graph`, `_define_alignment_graph`, the mapping module, and
 `session.run([loss, optimizer], feed_dict)` — on oracle/tf1_shim.py (a TensorFlow-1 graph interpreter on torch float64;
-TensorFlow itself is not installable here).  Runs only where /root/reference exists; the fixture it writes is what
-travels.  Per case: the variables' start values, every run's feeds, the fetched loss of every run and all variables
+TensorFlow itself is not installable here).  Runs with OPENEA_REFERENCE set to a checkout of the original project; the
+fixture it writes is what travels.  Per case: the variables' start values, every run's feeds, the fetched loss of every run and all variables
 after the last run.
 
-    python scripts/make_golden_path_i.py
+    OPENEA_REFERENCE=/path/to/OpenEA python scripts/make_golden_path_i.py
 """
 import importlib
 import json
@@ -17,10 +17,10 @@ import numpy as np
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 sys.path.insert(0, ROOT)
-sys.dont_write_bytecode = True          # never write into /root/reference
+sys.dont_write_bytecode = True          # never write into the reference checkout
 from oracle import tf1_shim  # noqa: E402
 
-REF_SRC = "/root/reference/src"
+REF_SRC = os.path.join(os.environ.get("OPENEA_REFERENCE", ""), "src")
 OUT = os.path.join(ROOT, "tests", "golden", "path_i_reference_graphs.npz")
 N_ENT, N_REL = 40, 6
 
@@ -433,7 +433,7 @@ def generate_alinet():
 
 if __name__ == "__main__":
     if not os.path.isdir(REF_SRC):
-        sys.exit("the reference is not present: goldens can only be generated where /root/reference exists")
+        sys.exit("set OPENEA_REFERENCE to a checkout of the original OpenEA: the goldens are generated from it")
     generate()
     generate_attre()
     generate_gcn_align()

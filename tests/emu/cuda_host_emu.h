@@ -29,6 +29,10 @@
 #define cudaMemcpyAsync(D, S, N, KIND, ST) (memcpy((D), (S), (N)), cudaSuccess)
 #define cudaStreamSynchronize(ST) (cudaSuccess)
 #define cudaFuncSetAttribute(...) (cudaSuccess)
+// An emulated kernel is a host function the real runtime does not know.  Asking the real runtime about it fails, and on
+// a machine with a GPU that failure would stay as the last error of the CUDA runtime the process shares with torch.
+// Answer with the one resident block per SM the grid sizing falls back to.
+#define cudaOccupancyMaxActiveBlocksPerMultiprocessor(N, ...) (*(N) = 1, cudaSuccess)
 /* launches and copies are synchronous and in program order: stream / event ordering is already satisfied */
 #define cudaStreamWaitEvent(...) (cudaSuccess)
 #define cudaEventRecord(...) (cudaSuccess)

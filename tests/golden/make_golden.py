@@ -1,7 +1,9 @@
 """Generate golden vectors from the REFERENCE ITSELF (its NumPy modules imported with TF stubbed).
 
-Run once in the authoring container (needs /root/reference):  python tests/golden/make_golden.py
-The .npz files it writes are committed; tests read them on any box (the GPU box has no /root/reference).
+Run with a checkout of the original project:  OPENEA_REFERENCE=/path/to/OpenEA python tests/golden/make_golden.py
+The .npz file it writes is committed; the tests read it and need no reference.  The similarity and CSLS matrices are
+stored for a seeded sample of rows (`<tag>_sim_rows`, first and last row included) to keep the file under 1 MB; the
+alignments, ranks and neighbour lists derived from the full matrices are stored whole.
 """
 import contextlib
 import io
@@ -23,6 +25,14 @@ def embeds(seed, n1, n2, d, noise=0.35):
     return e1, e2
 
 
+SIM_ROWS = {"a": 32, "b": 24}
+
+
+def sim_rows(tag, n1):
+    rows = np.random.default_rng(0).choice(np.arange(1, n1 - 1), SIM_ROWS[tag] - 2, replace=False)
+    return np.sort(np.concatenate([[0, n1 - 1], rows])).astype(np.int64)
+
+
 def main():
     ref = ref_adapter.load()
     out = {}
@@ -31,13 +41,14 @@ def main():
     for tag, seed, n1, n2, d in cases:
         e1, e2 = embeds(seed, n1, n2, d)
         out["%s_e1" % tag], out["%s_e2" % tag] = e1, e2
+        rows = out["%s_sim_rows" % tag] = sim_rows(tag, n1)
         for metric, norm in (("inner", False), ("inner", True), ("cosine", False), ("euclidean", False), ("manhattan", False)):
             with contextlib.redirect_stdout(quiet):
                 s = ref.similarity.sim(e1, e2, metric=metric, normalize=norm, csls_k=0)
                 sc = ref.similarity.sim(e1, e2, metric=metric, normalize=norm, csls_k=10)
             key = "%s_%s_%d" % (tag, metric, int(norm))
-            out[key + "_sim"] = s.astype(np.float32)
-            out[key + "_csls"] = sc.astype(np.float32)
+            out[key + "_sim"] = s[rows].astype(np.float32)
+            out[key + "_csls"] = sc[rows].astype(np.float32)
             for csls_k in (0, 10):
                 with contextlib.redirect_stdout(quiet):
                     pairs, hits1, mr, mrr = ref.alignment.greedy_alignment(e1, e2, [1, 5, 10, 50], 1, metric, norm, csls_k, True)

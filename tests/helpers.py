@@ -1,7 +1,80 @@
 """Shared test helpers: float64 torch-autograd statement of the triple-scoring graph (an independent
-derivation used to check the C oracle's hand-written backward) and seeded batch generators."""
+derivation used to check the C oracle's hand-written backward), seeded batch generators, and the recorded results of
+the original OpenEA functions the host ports are compared with."""
+import hashlib
+import json
+import numbers
+import os
+from collections.abc import Mapping, Set
+
 import numpy as np
 import torch
+
+GOLDEN = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden")
+
+
+def canonical(x):
+    """Text form of a result that is equal for two results exactly when Python's == holds between them (dicts and sets
+    in sorted order, integral floats as ints, NumPy scalars and arrays as Python values)."""
+    if isinstance(x, Mapping):
+        return "{" + ",".join(sorted(canonical(k) + ":" + canonical(v) for k, v in x.items())) + "}"
+    if isinstance(x, Set):
+        return "set(" + ",".join(sorted(canonical(e) for e in x)) + ")"
+    if isinstance(x, tuple):
+        return "(" + ",".join(canonical(e) for e in x) + ")"
+    if isinstance(x, (list, np.ndarray)):
+        return "[" + ",".join(canonical(e) for e in x) + "]"
+    if isinstance(x, (bool, np.bool_)):
+        return repr(bool(x))
+    if isinstance(x, numbers.Integral):
+        return str(int(x))
+    if isinstance(x, numbers.Real):
+        f = float(x)
+        return str(int(f)) if f.is_integer() else repr(f)
+    if isinstance(x, str) or x is None:
+        return repr(x)
+    raise TypeError("no canonical form for %r" % type(x))
+
+
+def digest(x):
+    return hashlib.sha256(canonical(x).encode("utf8")).hexdigest()
+
+
+class ReferenceRecord:
+    """What the original OpenEA functions returned on a test's inputs, stored as tests/golden/<name>.json (SHA-256 of
+    the canonical form of results compared with ==) and tests/golden/<name>.npz (arrays compared with a tolerance).
+
+    With OPENEA_REFERENCE set to a checkout of the original project, `reference` callables are run live, the test's
+    comparison is made against the live result, and the record is rewritten; otherwise the stored record is used."""
+
+    def __init__(self, name):
+        self.json_path = os.path.join(GOLDEN, name + ".json")
+        self.npz_path = os.path.join(GOLDEN, name + ".npz")
+        self.live = bool(os.environ.get("OPENEA_REFERENCE"))
+        self.digests, self.arrays = {}, {}
+        if os.path.exists(self.json_path):
+            with open(self.json_path) as f:
+                self.digests = json.load(f)
+        if os.path.exists(self.npz_path):
+            with np.load(self.npz_path) as z:
+                self.arrays = {k: z[k] for k in z.files}
+
+    def equal(self, key, mine, reference):
+        """mine == the reference's result (`reference()` is only called when recording)."""
+        if self.live:
+            want = reference()
+            self.digests[key] = digest(want)
+            with open(self.json_path, "w") as f:
+                json.dump(self.digests, f, indent=0, sort_keys=True)
+            return mine == want
+        return digest(mine) == self.digests[key]
+
+    def array(self, key, reference):
+        """The reference's numeric result as an array (`reference()` is only called when recording)."""
+        if self.live:
+            self.arrays[key] = np.asarray(reference())
+            np.savez_compressed(self.npz_path, **self.arrays)
+        return self.arrays[key]
 
 
 def torch_triple_loss(ent, rel, pos, neg, loss, loss_norm, ent_norm, rel_norm, margin=0.0, neg_margin=0.0,

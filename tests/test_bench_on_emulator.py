@@ -6,6 +6,7 @@ import os
 import subprocess
 import sys
 
+import numpy as np
 import pytest
 
 from tests.emu import build_emu
@@ -22,8 +23,9 @@ def run(*args, timeout=600):
     return res.stdout.strip().splitlines()
 
 
-def test_bench_line_contract_on_the_emulator():
-    line = json.loads(run("bench", "--workload", "micro", "--steps", "3", "--warmup", "3", "--no-cpu-baseline")[-1])
+def test_bench_line_contract_on_the_emulator(tmp_path):
+    line = json.loads(run("bench", "--workload", "micro", "--steps", "3", "--warmup", "3", "--no-cpu-baseline",
+                          "--dump-outputs", str(tmp_path / "out"))[-1])
     for key in ("metric", "value", "unit", "n_gpus", "steps", "warmup", "ms_per_step", "higher_is_better", "scaling",
                 "vs_baseline", "dtype", "data", "config", "roofline", "e2e", "cpu_baseline", "clocks", "gpu_launches"):
         assert key in line, key
@@ -33,6 +35,14 @@ def test_bench_line_contract_on_the_emulator():
     assert set(("bound", "achieved", "peak", "unit", "frac", "traffic")) <= set(roof) and roof["bound"] == "hbm"
     e2e = line["e2e"]
     assert e2e["value"] > 0 and e2e["h2d_bytes_per_step"] == 12 * 48 * 4 and e2e["d2h_bytes_per_step"] == 8
+    assert e2e["steps"] == 3
+    dumped = {f[:-4]: np.load(tmp_path / "out" / f) for f in os.listdir(tmp_path / "out")}
+    assert set(dumped) == {"last_step_loss", "entity_embeddings_sampled", "entity_adagrad_sampled", "relation_embeddings",
+                           "relation_adagrad"}
+    assert all(a.dtype in (np.float32, np.float64) and np.isfinite(a).all() for a in dumped.values())
+    assert dumped["last_step_loss"].shape == (1,) and dumped["last_step_loss"][0] > 0
+    assert dumped["entity_embeddings_sampled"].shape == dumped["entity_adagrad_sampled"].shape
+    assert sum(a.nbytes for a in dumped.values()) <= 64 << 20
     csls = line["csls"]
     assert csls["value"] > 0 and csls["e2e"]["value"] > 0 and csls["cpu_baseline"]["value"] > 0 and csls["hits1"] > 0
 

@@ -40,10 +40,11 @@ def finding_cpu(monkeypatch):
 def test_emulated_sim_matrix_and_csls_equal_the_reference_golden(finding_cpu, tag, metric, norm):
     e1, e2 = GOLD[tag + "_e1"], GOLD[tag + "_e2"]
     key = "%s_%s_%d" % (tag, metric, norm)
+    rows = GOLD[tag + "_sim_rows"]
     got = finding_cpu.sim(e1, e2, metric, bool(norm), 0).numpy()
-    np.testing.assert_allclose(got, GOLD[key + "_sim"], rtol=2e-5, atol=3e-5)
+    np.testing.assert_allclose(got[rows], GOLD[key + "_sim"], rtol=2e-5, atol=3e-5)
     got = finding_cpu.sim(e1, e2, metric, bool(norm), 10).numpy()
-    np.testing.assert_allclose(got, GOLD[key + "_csls"], rtol=2e-5, atol=1e-4)
+    np.testing.assert_allclose(got[rows], GOLD[key + "_csls"], rtol=2e-5, atol=1e-4)
 
 
 @pytest.mark.parametrize("materialize", [True, False])

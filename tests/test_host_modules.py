@@ -1,6 +1,6 @@
 """CPU tests of the host-side mirror of the reference interface: args, task_divide, batch slicing, id
-assignment, dataset loading (against goldens generated from the reference and, where present, the live
-reference), the host sampler's rules, Gale-Shapley, early_stop, and the `openea` drop-in import surface."""
+assignment, dataset loading (against goldens generated from the reference: stored vectors and recorded results of its
+read_kgs_from_folder), the host sampler's rules, Gale-Shapley, early_stop, and the `openea` drop-in import surface."""
 import ast
 import contextlib
 import io
@@ -12,8 +12,10 @@ import numpy as np
 import pytest
 
 from oracle import ref_adapter
+from tests.helpers import ReferenceRecord
 
 GOLD = np.load(os.path.join(os.path.dirname(__file__), "golden", "finding_golden.npz"))
+REC = ReferenceRecord("reference_host_modules")
 
 
 def test_args_loader(tmp_path):
@@ -144,6 +146,8 @@ def test_openea_dropin_import_surface():
 
 def _reference_kgs(folder, modes):
     """read_kgs_from_folder of the live reference (TensorFlow stubbed) for the given id modes."""
+    if not REC.live:
+        return None
     import importlib
     import sys
     import types
@@ -165,10 +169,9 @@ def _reference_kgs(folder, modes):
         sys.modules.update(saved)
 
 
-@pytest.mark.skipif(not ref_adapter.available(), reason="/root/reference not present on this box")
 @pytest.mark.parametrize("loader", ["arrays", "containers", "arrays-cached"])
 def test_dataset_loading_equals_live_reference(tmp_path, monkeypatch, loader):
-    """Full read_kgs_from_folder equivalence with the live reference on a synthetic folder, in all three id modes, for
+    """Full read_kgs_from_folder equivalence with the reference on a synthetic folder, in all three id modes, for
     the array-backed loader (fresh parse and binary cache) and the container-based loader: id dicts, triple sets and
     lists incl. swap triples, every derived dict, vocabularies, counts, links, URI-level KGs."""
     from openea_b200.modules.load import fast
@@ -188,37 +191,34 @@ def test_dataset_loading_equals_live_reference(tmp_path, monkeypatch, loader):
         assert log.getvalue().count("loaded from cache") == 3
     assert isinstance(mine["mapping"], fast.ArrayKGs) == (loader != "containers")
     theirs = _reference_kgs(folder, modes)
-    for m in mine:
-        a, b = mine[m], theirs[m]
-        assert a.entities_num == b.entities_num and a.relations_num == b.relations_num and a.attributes_num == b.attributes_num
+
+    def facts(k):
+        f = {"nums": (k.entities_num, k.relations_num, k.attributes_num)}
         for side in ("kg1", "kg2", "uri_kg1", "uri_kg2"):
-            ka, kb = getattr(a, side), getattr(b, side)
+            g = getattr(k, side)
+            names = ["relation_triples_set", "attribute_triples_set", "local_relation_triples_set", "rt_dict", "hr_dict",
+                     "av_dict", "entity_relations_dict", "entity_attributes_dict", "entities_set", "relations_set",
+                     "attributes_set", "entities_num", "relations_num", "attributes_num", "relation_triples_num",
+                     "local_relation_triples_num", "attribute_triples_num", "local_attribute_triples_num"]
             if not side.startswith("uri"):
-                assert ka.entities_id_dict == kb.entities_id_dict and ka.relations_id_dict == kb.relations_id_dict
-                assert ka.attributes_id_dict == kb.attributes_id_dict
-                assert ka.sup_relation_triples_set == kb.sup_relation_triples_set
-                assert ka.sup_attribute_triples_set == kb.sup_attribute_triples_set
-            assert ka.relation_triples_set == kb.relation_triples_set and ka.attribute_triples_set == kb.attribute_triples_set
-            assert ka.local_relation_triples_set == kb.local_relation_triples_set
+                names += ["entities_id_dict", "relations_id_dict", "attributes_id_dict", "sup_relation_triples_set",
+                          "sup_attribute_triples_set"]
+            for name in names:
+                f[side + "." + name] = getattr(g, name)
             for lst in ("relation_triples_list", "local_relation_triples_list", "attribute_triples_list",
                         "local_attribute_triples_list", "entities_list", "relations_list", "attributes_list"):
-                la, lb = getattr(ka, lst), getattr(kb, lst)
-                assert len(la) == len(lb) and set(la) == set(lb), (m, side, lst)
-            for dct in ("rt_dict", "hr_dict", "av_dict", "entity_relations_dict", "entity_attributes_dict"):
-                assert getattr(ka, dct) == getattr(kb, dct), (m, side, dct)
-            for st in ("entities_set", "relations_set", "attributes_set"):
-                assert getattr(ka, st) == getattr(kb, st), (m, side, st)
-            for num in ("entities_num", "relations_num", "attributes_num", "relation_triples_num",
-                        "local_relation_triples_num", "attribute_triples_num", "local_attribute_triples_num"):
-                assert getattr(ka, num) == getattr(kb, num), (m, side, num)
+                f[side + "." + lst] = (len(getattr(g, lst)), set(getattr(g, lst)))
         for part in ("train", "valid", "test"):
-            assert getattr(a, part + "_links") == getattr(b, part + "_links")
-            assert getattr(a, part + "_entities1") == getattr(b, part + "_entities1")
-            assert getattr(a, "uri_%s_links" % part) == getattr(b, "uri_%s_links" % part)
-        assert set(a.useful_entities_list1) == set(b.useful_entities_list1)
+            for name in (part + "_links", part + "_entities1", "uri_%s_links" % part):
+                f[name] = getattr(k, name)
+        f["useful_entities_list1"] = set(k.useful_entities_list1)
+        return f
+    for m in mine:
+        want = facts(theirs[m]) if REC.live else None
+        for key, val in facts(mine[m]).items():
+            assert REC.equal("tiny/%s/%s" % (m, key), val, lambda: want[key]), (m, key)
 
 
-@pytest.mark.skipif(not ref_adapter.available(), reason="/root/reference not present on this box")
 @pytest.mark.parametrize("case", ["clean", "dirty"])
 def test_array_loader_edge_cases_equal_live_reference(tmp_path, monkeypatch, case):
     """Hand-written folder: duplicate lines, padded fields, values with a trailing '.', an entity that only carries
@@ -246,16 +246,21 @@ def test_array_loader_edge_cases_equal_live_reference(tmp_path, monkeypatch, cas
     assert isinstance(mine["mapping"], fast.ArrayKGs) == (case == "clean")
     assert ("array-backed loader not applicable" in log.getvalue()) == (case == "dirty")
     theirs = _reference_kgs(folder, modes)
-    for m in modes:
-        a, b = mine[m], theirs[m]
-        assert (a.entities_num, a.relations_num, a.attributes_num) == (b.entities_num, b.relations_num, b.attributes_num)
+
+    def facts(k):
+        f = {"nums": (k.entities_num, k.relations_num, k.attributes_num)}
         for side in ("kg1", "kg2"):
-            ka, kb = getattr(a, side), getattr(b, side)
             for name in ("entities_id_dict", "relations_id_dict", "attributes_id_dict", "relation_triples_set",
                          "attribute_triples_set", "sup_relation_triples_set", "sup_attribute_triples_set", "rt_dict",
                          "hr_dict", "av_dict", "entity_attributes_dict", "entities_set"):
-                assert getattr(ka, name) == getattr(kb, name), (m, side, name)
-        assert a.train_links == b.train_links and a.valid_links == b.valid_links and a.test_links == b.test_links
+                f[side + "." + name] = getattr(getattr(k, side), name)
+        for name in ("train_links", "valid_links", "test_links"):
+            f[name] = getattr(k, name)
+        return f
+    for m in modes:
+        want = facts(theirs[m]) if REC.live else None
+        for key, val in facts(mine[m]).items():
+            assert REC.equal("edge-%s/%s/%s" % (case, m, key), val, lambda: want[key]), (m, key)
 
 
 def test_array_loader_refuses_what_only_the_container_loader_covers(tmp_path):
@@ -369,20 +374,17 @@ def test_pair_set_behaves_like_the_reference_set():
 
 
 def test_galeshapley_port_equals_the_reference_function():
-    """The host restatement of galeshapley against the reference's own function (imported live with TF stubbed) on
+    """The host restatement of galeshapley against the reference's own function (recorded with TF stubbed) on
     random preference structures, including max_iteration cut-offs that stop before everybody is matched."""
-    from oracle import ref_adapter
-    if not ref_adapter.available():
-        pytest.skip("reference sources not present")
     import copy
     from openea_b200.modules.finding.alignment import arg_sort, galeshapley
-    ref = ref_adapter.load().alignment
+    ref = ref_adapter.load().alignment if REC.live else None
     rng = np.random.default_rng(5)
     for n1, n2, cut in ((12, 12, 100), (20, 15, 100), (15, 20, 3), (30, 30, 2)):
         s = rng.standard_normal((n1, n2)).astype(np.float32)
         a = arg_sort(list(range(n1)), s, "x_", "y_"); b = arg_sort(list(range(n2)), s.T, "y_", "x_")
         if n1 > n2 and cut >= n2:
             continue      # more suitors than reviewers and unlimited rounds: the reference runs lists empty (IndexError)
-        want = ref.galeshapley(copy.deepcopy(a), copy.deepcopy(b), cut)
         got = galeshapley(copy.deepcopy(a), copy.deepcopy(b), cut)
-        assert got == want, (n1, n2, cut)
+        assert REC.equal("galeshapley/%d-%d-%d" % (n1, n2, cut), got,
+                         lambda: ref.galeshapley(copy.deepcopy(a), copy.deepcopy(b), cut)), (n1, n2, cut)

@@ -1,6 +1,6 @@
 """CPU: IPTransE's host / index layer (openea_b200/approaches/iptranse.py) — the two-step path table against a
-brute-force statement of iptranse.py:98-121 and against the reference's own pandas source (where /root/reference
-exists), the triples of latent aligned entities against the reference's dict walk, and the whole approach
+brute-force statement of iptranse.py:98-121 and against recorded results of the reference's own pandas source, the
+triples of latent aligned entities against the reference's dict walk, and the whole approach
 (PTransE epochs + an alignment epoch) on the CPU warp emulator."""
 import collections
 import re
@@ -11,7 +11,10 @@ import torch
 
 from openea_b200.approaches import iptranse as ipt
 from oracle import reference_source as ref_src
+from tests.helpers import ReferenceRecord
 from tests.test_emu_triple_core import cpu_engine      # noqa: F401  (fixture: the engine over the emulated library)
+
+REC = ReferenceRecord("reference_iptranse")
 
 
 def random_kg(rng, n_ent, n_rel, n_tri):
@@ -45,15 +48,15 @@ def test_two_step_paths_equal_a_brute_force_join(seed, n_ent, n_rel, n_tri):
     assert ipt.two_step_paths(np.zeros((0, 3), np.int64))[0].shape == (0, 3)
 
 
-@pytest.mark.skipif(ref_src.iptranse_helpers() is None, reason="/root/reference not present on this box")
 def test_two_step_paths_and_latent_triples_equal_the_reference_source():
-    ref = ref_src.iptranse_helpers()
+    ref = ref_src.iptranse_helpers() if REC.live else None
     rng = np.random.default_rng(5)
     tri = random_kg(rng, 60, 7, 500)
-    want = collections.Counter((int(a), int(b), int(c), float(w)) for a, b, c, w in
-                               ref["generate_2steps_path"]([tuple(int(v) for v in t) for t in tri]))
     rows, w = ipt.two_step_paths(tri)
-    assert collections.Counter((int(a), int(b), int(c), float(x)) for (a, b, c), x in zip(rows, w)) == want
+    assert REC.equal("generate_2steps_path",
+                     collections.Counter((int(a), int(b), int(c), float(x)) for (a, b, c), x in zip(rows, w)),
+                     lambda: collections.Counter((int(a), int(b), int(c), float(w)) for a, b, c, w in
+                                                 ref["generate_2steps_path"]([tuple(int(v) for v in t) for t in tri])))
 
     # triples of latent aligned entities: kg1 over ids 0..59, kg2 over 60..119; several kg1 entities may share a partner
     tri2 = random_kg(rng, 60, 7, 400) + np.array([60, 0, 60])
@@ -68,14 +71,15 @@ def test_two_step_paths_and_latent_triples_equal_the_reference_source():
     ents1 = rng.choice(60, 25, replace=False)
     ents2 = rng.integers(60, 120, 25)
     ws = rng.random(25).astype(np.float32)
-    want = ref["generate_triples_of_latent_ents"](KGs, [int(e) for e in ents1], [int(e) for e in ents2], [float(x) for x in ws])
     t1, t2 = torch.as_tensor(tri.astype(np.int32)), torch.as_tensor(tri2.astype(np.int32))
     e1, e2, w = torch.as_tensor(ents1), torch.as_tensor(ents2), torch.as_tensor(ws)
     a, wa = ipt.latent_triples(ipt._by_column(t1, 0, 120), ipt._by_column(t1, 2, 120), e1, e2, w)
     b, wb = ipt.latent_triples(ipt._by_column(t2, 0, 120), ipt._by_column(t2, 2, 120), e2, e1, w)
     got_t, got_w = ipt.distinct_weighted(torch.cat([a, b]), torch.cat([wa, wb]), 120, 7)
     got = {(int(h), int(r), int(t), float(x)) for (h, r, t), x in zip(got_t.tolist(), got_w.tolist())}
-    assert got == want and len(got) == got_t.shape[0]
+    assert REC.equal("generate_triples_of_latent_ents", got, lambda: ref["generate_triples_of_latent_ents"](
+        KGs, [int(e) for e in ents1], [int(e) for e in ents2], [float(x) for x in ws]))
+    assert len(got) == got_t.shape[0]
 
 
 def test_iptranse_lifecycle_on_the_emulator(cpu_engine, monkeypatch, tmp_path, capsys):

@@ -1,5 +1,5 @@
 """CPU: pin the NumPy oracle for path (iii) against golden vectors generated FROM THE REFERENCE ITSELF
-(tests/golden/make_golden.py) and, where /root/reference is present, against the live reference functions."""
+(tests/golden/make_golden.py) and against results the reference functions returned on a further seed."""
 import ast
 import contextlib
 import io
@@ -10,7 +10,9 @@ import pytest
 
 from oracle import finding as orf
 from oracle import ref_adapter
+from tests.helpers import ReferenceRecord
 
+REC = ReferenceRecord("reference_oracle_finding")
 GOLD = np.load(os.path.join(os.path.dirname(__file__), "golden", "finding_golden.npz"))
 METRICS = [("inner", 0), ("inner", 1), ("cosine", 0), ("euclidean", 0), ("manhattan", 0)]
 
@@ -20,10 +22,11 @@ METRICS = [("inner", 0), ("inner", 1), ("cosine", 0), ("euclidean", 0), ("manhat
 def test_sim_and_csls_match_reference(tag, metric, norm):
     e1, e2 = GOLD[tag + "_e1"], GOLD[tag + "_e2"]
     key = "%s_%s_%d" % (tag, metric, norm)
+    rows = GOLD[tag + "_sim_rows"]
     s = orf.sim(e1, e2, metric, bool(norm), 0)
-    np.testing.assert_allclose(s, GOLD[key + "_sim"], rtol=2e-5, atol=2e-5)
+    np.testing.assert_allclose(s[rows], GOLD[key + "_sim"], rtol=2e-5, atol=2e-5)
     sc = orf.sim(e1, e2, metric, bool(norm), 10)
-    np.testing.assert_allclose(sc, GOLD[key + "_csls"], rtol=2e-5, atol=6e-5)
+    np.testing.assert_allclose(sc[rows], GOLD[key + "_csls"], rtol=2e-5, atol=6e-5)
 
 
 @pytest.mark.parametrize("tag", ["a", "b"])
@@ -72,15 +75,19 @@ def test_csls_known_answer_3x4():
     np.testing.assert_allclose(orf.csls_sim(s, 2), want)
 
 
-@pytest.mark.skipif(not ref_adapter.available(), reason="/root/reference not present on this box")
 def test_live_reference_agrees_on_fresh_seed():
-    ref = ref_adapter.load()
+    ref = ref_adapter.load() if REC.live else None
     rng = np.random.default_rng(2024)
     e2 = rng.standard_normal((150, 64)).astype(np.float32)
     e1 = (e2[:120] + 0.4 * rng.standard_normal((120, 64))).astype(np.float32)
     for metric, norm, k in (("inner", True, 10), ("manhattan", False, 5), ("euclidean", False, 0)):
-        with contextlib.redirect_stdout(io.StringIO()):
-            want, h1, mr, mrr = ref.alignment.greedy_alignment(e1, e2, [1, 5], 1, metric, norm, k, True)
+        def reference():
+            with contextlib.redirect_stdout(io.StringIO()):
+                want, h1, mr, mrr = ref.alignment.greedy_alignment(e1, e2, [1, 5], 1, metric, norm, k, True)
+            return np.array(sorted(want), dtype=np.float64).reshape(-1), np.array([h1, mr, mrr], dtype=np.float64)
+        key = "%s-%d-%d" % (metric, norm, k)
+        want = REC.array(key + "/pairs", lambda: reference()[0]).astype(np.int64).reshape(-1, 2)
+        h1, mr, mrr = REC.array(key + "/stats", lambda: reference()[1])
         got, hits, gmr, gmrr = orf.greedy_alignment(e1, e2, [1, 5], metric, norm, k)
         assert got == {(int(i), int(j)) for i, j in want} and hits[0] == pytest.approx(h1)
         assert gmr == pytest.approx(mr) and gmrr == pytest.approx(mrr)
